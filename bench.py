@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the pylops-mpi hot path on B200 (contract: see the task brief).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras] [--dump-outputs DIR]
 
 Headline (BASELINE.json metric "... GB/s (FirstDerivative)"): one *step* is one
 ``MPIFirstDerivative.matvec`` (centered, order 3, float32) over the (65536, 8192)
@@ -16,6 +16,10 @@ world size (``parity`` in the line; a failure aborts the timing).
 ``secondary`` = the MatrixMult half of BASELINE's metric (GF/s on the 32768^2
 bf16 config, with its own roofline and a 256-sampled-rows parity check) and the
 weak-scaling curve of the stencil; ``extra`` = the other BASELINE configs.
+
+``--dump-outputs DIR`` writes, after the timed steps, a fixed seeded sample of what the last timed step returned
+(whole rows of the (65536, 8192) result, float32) and their row indices (float64) as DIR/*.npy.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 ``--impl reference`` times the reference's CPU algorithm for the same operator
 on the same global workload (the NumPy restatement in oracle/, one OS process
@@ -46,6 +50,7 @@ NCOLS = 8192
 METRIC = "MPIFirstDerivative matvec GB/s (algorithmic bytes, centered-3 float32)"
 METRIC2 = "MPIMatrixMult matvec GF/s (bf16 -> fp32, 32768 x 32768, M = 4096)"
 HBM_FALLBACK = 6650.0
+DUMP_ROWS = 1024               # rows of the headline output written by --dump-outputs: 1024 x 8192 float32 = 32 MiB
 
 
 def load_peaks():
@@ -237,6 +242,24 @@ def time_loop(fn, steps, warmup, comm=None):
     return ms
 
 
+def dump_outputs(out_dir, y, comm, nloc):
+    """write DUMP_ROWS rows of the headline output ``y`` (global shape (GLOBAL_ROWS, NCOLS)): the first and last row
+    of every rank's block, where the halo exchange acts, and the rest drawn with a fixed seed"""
+    import torch
+    rank, size = comm.Get_rank(), comm.Get_size()
+    edges = {r * nloc for r in range(size)} | {(r + 1) * nloc - 1 for r in range(size)}
+    pool = np.setdiff1d(np.arange(GLOBAL_ROWS), sorted(edges))
+    rows = np.union1d(sorted(edges), np.random.default_rng(0).choice(pool, DUMP_ROWS - len(edges), replace=False))
+    mine = rows[(rows >= rank * nloc) & (rows < (rank + 1) * nloc)]
+    yl = y.local_array.reshape(nloc, NCOLS)
+    local = yl[torch.as_tensor(mine - rank * nloc, device=yl.device)].cpu().numpy()
+    parts = comm.allgather(local)
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "first_derivative_y_rows.npy"), np.concatenate(parts).astype(np.float32))
+        np.save(os.path.join(out_dir, "first_derivative_y_row_index.npy"), rows.astype(np.float64))
+
+
 def numa_bind_to_gpu(dev: int):
     """pin this process (and, by first touch, its pinned host buffers) to the NUMA node the GPU hangs off:
     with 8 ranks the e2e host<->device pipelines otherwise cross the inter-socket link for half of the GPUs"""
@@ -331,6 +354,8 @@ def run_gpu_arm(args):
     enqueue_ms = time_loop.last_enqueue_ms     # host time to enqueue one step (GPU-bound if << ms_per_step)
     value = bytes_loc * size * args.steps / (ms * 1e-3) / 1e9
     fused_halo = size > 1 and comm.halo is not None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, holder["y"], comm, nloc)
 
     # ---- roofline of the dominant kernel: live CUDA-event timing of the kernel alone --------
     xl = x.local_array
@@ -766,6 +791,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-check", action="store_true", help="skip the multi-rank parity preamble")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of the last step's output to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":

@@ -1,11 +1,12 @@
-"""Generate golden fixtures by running the REAL reference (/root/reference,
-imported unmodified) under the in-process MPI shim in tests/golden/refshim/.
+"""Generate golden fixtures by running the REAL reference (a pylops-mpi source
+checkout, imported unmodified) under the in-process MPI shim in tests/golden/refshim/.
 
-    python tests/golden/make_golden.py            # writes tests/golden/reference_golden.npz
+    PYLOPS_MPI_REFERENCE=<pylops-mpi checkout> python tests/golden/make_golden.py
+                                                  # writes tests/golden/reference_golden.npz
 
-Runs only in the build container (the GPU box has no /root/reference); the
-.npz it writes is committed and is what tests/test_golden.py checks the oracle
-and the CUDA path against.  Third-party ``pylops`` is absent from the image.  On
+Needs the reference checkout; the tests do not.  The .npz it writes (in the compact
+form of tests/golden_store.py) is committed and is what tests/test_golden.py checks
+the oracle and the CUDA path against.  Third-party ``pylops`` is absent from the image.  On
 the hot path its only arithmetic (the dense block ``A @ x``) is restated in
 refshim/pylops; mpi4py is replaced by threads.  Everything else -- partition
 bookkeeping, @reshaped, ghost cells, the stencils, BlockDiag/VStack/MatrixMult/
@@ -27,8 +28,10 @@ import types
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("PYLOPS_MPI_REFERENCE", "/root/reference")
+REF = os.environ.get("PYLOPS_MPI_REFERENCE", "")
 sys.path.insert(0, os.path.join(HERE, "refshim"))
+sys.path.insert(0, os.path.dirname(HERE))
+import golden_store  # noqa: E402
 
 
 def load_reference():
@@ -63,6 +66,8 @@ def load_reference():
 
 
 def main():
+    if not os.path.isdir(os.path.join(REF, "pylops_mpi")):
+        raise SystemExit("set PYLOPS_MPI_REFERENCE to a pylops-mpi source checkout")
     from mpi4py import MPI
     import pylops
     pkg, mods = load_reference()
@@ -383,7 +388,7 @@ def main():
                     assert np.array_equal(res[r]["y"], res[0]["y"]) and np.array_equal(res[r]["xa"], res[0]["xa"])
 
     path = os.path.join(HERE, os.environ.get("GOLDEN_OUT", "reference_golden.npz"))
-    np.savez_compressed(path, **out)
+    golden_store.save(path, out)
     print(f"wrote {path}: {len(out)} arrays, {os.path.getsize(path) / 1e6:.2f} MB")
 
 

@@ -1,8 +1,11 @@
 """Golden-vector tests.  tests/golden/reference_golden.npz was produced by the
-REAL reference code (imported from /root/reference under the in-process MPI shim,
-tests/golden/make_golden.py).  Here:
+REAL reference code (pylops-mpi, imported unmodified under the in-process MPI shim,
+tests/golden/make_golden.py) and is stored compactly (tests/golden_store.py): inputs
+are redrawn here from their seeds and pinned by digest, larger outputs are kept as
+digest + samples + weighted sum.  Here:
   * CPU (not gpu): the oracle must reproduce every fixture -> the oracle is pinned;
-  * GPU: the CUDA path (world size 1) must reproduce the gathered fixtures.
+  * GPU: the CUDA path (world size 1) must reproduce the gathered fixtures, and every
+    entry must match the oracle (pinned to the same fixtures by the CPU tests).
 """
 import ast
 import math
@@ -12,11 +15,12 @@ import re
 import numpy as np
 import pytest
 
+import golden_store
 import pylops_mpi_oracle as o
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GOLD = np.load(os.path.join(HERE, "golden", "reference_golden.npz"), allow_pickle=False)
-KEYS = list(GOLD.keys())
+GOLD = golden_store.Golden(os.path.join(HERE, "golden", "reference_golden.npz"))
+KEYS = GOLD.keys()
 
 
 def cases(prefix, depth):
@@ -30,13 +34,17 @@ def cases(prefix, depth):
     return seen
 
 
-def ranks_of(case, name):
-    out = []
-    r = 0
-    while f"{case}/r{r}/{name}" in GOLD:
-        out.append(GOLD[f"{case}/r{r}/{name}"])
-        r += 1
-    return out
+def rec(case, name):
+    return GOLD.record(f"{case}/{name}")
+
+
+def normal_input(seed, n, dtype):
+    """input of the stencil fixtures, drawn as make_golden draws it"""
+    rng = np.random.default_rng(seed)
+    x = rng.normal(0, 10, n).astype(dtype)
+    if np.issubdtype(dtype, np.complexfloating):
+        x = x + 1j * rng.normal(0, 10, n)
+    return x
 
 
 FD_CASES = cases("fd", 7)
@@ -49,11 +57,22 @@ def parse_fd(case):
     return int(P[1:]), ast.literal_eval(dims), float(h[1:]), kind, int(order), bool(int(e[1:])), np.dtype(dt)
 
 
+def fd_oracle(case):
+    """the fixture's input (checked against the reference's) and the oracle's per-rank outputs"""
+    P, dims, h, kind, order, edge, dt = parse_fd(case)
+    x = normal_input(7, int(np.prod(dims)), dt)
+    rec(case, "x").check(x)
+    y = o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, False, dtype=dt)
+    ya = o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, True, dtype=dt)
+    return x, y, ya
+
+
 def test_fixture_inventory():
     assert len(FD_CASES) == 4 * 5 * 4 * 2 * 2
     assert len(cases("array", 4)) == 16 and len(cases("stack", 4)) == 12
     assert len(cases("mm", 5)) == 30 and len(cases("fredholm", 5)) == 24
     assert "config1/y" in GOLD
+    assert "array/P1/(50, 51)/ax1/r0/dot" in GOLD and "array/P1/(50, 51)/ax1/r1/dot" not in GOLD
 
 
 # ---------------------------------------------------------------------------------------------
@@ -68,26 +87,28 @@ def test_oracle_first_derivative(case):
             o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, False, dtype=dt)
             o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, True, dtype=dt)
         return
-    x = GOLD[case + "/x"]
-    y = o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, False, dtype=dt)
-    ya = o.first_derivative(o.to_dist(x, P), dims, h, kind, edge, order, True, dtype=dt)
-    for r, (gy, gya) in enumerate(zip(ranks_of(case, "y"), ranks_of(case, "ya"))):
-        np.testing.assert_array_equal(y[r], gy.ravel())       # same NumPy ops -> bit-exact
-        np.testing.assert_array_equal(ya[r], gya.ravel())
+    x, y, ya = fd_oracle(case)
+    rec(case, "y").check(y)          # same NumPy ops -> bit-exact
+    rec(case, "ya").check(ya)
 
 
-def test_oracle_config1():
+def config1_oracle():
     x = np.zeros((11, 21))
     x[5, 10] = 1.0
     y = np.concatenate(o.first_derivative(o.to_dist(x.ravel(), 2), (11, 21)))
-    assert np.array_equal(y.reshape(11, 21), GOLD["config1/y"])
     mv = lambda a: o.SimArray(o.first_derivative(a.locs, (11, 21)))                   # noqa: E731
     rmv = lambda a: o.SimArray(o.first_derivative(a.locs, (11, 21), adjoint=True))    # noqa: E731
     xo, istop, iit, r1, r2, cost = o.cgls(mv, rmv, mv(o.SimArray(o.to_dist(x.ravel(), 2))),
                                           o.SimArray([np.zeros(126), np.zeros(105)]), niter=10, tol=0.0)
+    return y, xo.asarray(), istop, iit, cost
+
+
+def test_oracle_config1():
+    y, xo, istop, iit, cost = config1_oracle()
+    GOLD.record("config1/y").check(y.reshape(11, 21))
     assert iit == int(GOLD["config1/iit"]) and istop == int(GOLD["config1/istop"])
     np.testing.assert_allclose(cost, GOLD["config1/cost"], rtol=1e-12, atol=1e-30)
-    np.testing.assert_allclose(xo.asarray(), GOLD["config1/xinv"], rtol=1e-12, atol=1e-30)
+    GOLD.record("config1/xinv").check(xo, rtol=1e-12, atol=1e-30)
 
 
 @pytest.mark.parametrize("case", cases("array", 4))
@@ -105,15 +126,15 @@ def test_oracle_distributed_array(case):
         assert [tuple(s) for s in g("local_shapes")] == o.local_shapes(shape, P, o.SCATTER, axis)
         np.testing.assert_allclose(o.dot(al, bl)[r], g("dot"), rtol=1e-14)
         np.testing.assert_allclose(o.dot(al, bl, vdot=True)[r], g("vdot"), rtol=1e-14)
-        np.testing.assert_array_equal(a + b, g("add"))
         for o_ in (1, 2, np.inf, -np.inf, 0, 3):
             np.testing.assert_allclose(o.norm(al, o_)[r], g(f"norm{o_}"), rtol=1e-14)
         np.testing.assert_allclose(o.dot([a] * P, [a] * P, partition=o.BROADCAST)[r], g("bdot"), rtol=1e-14)
         if P >= 2:
             np.testing.assert_allclose(o.dot(al, al, mask=mask)[r], g("mdot"), rtol=1e-14)
             np.testing.assert_allclose(o.norm(al, 1, mask=mask)[r], g("mnorm"), rtol=1e-14)
-        if f"{case}/r{r}/ghost" in GOLD:
-            np.testing.assert_array_equal(o.add_ghost_cells(al, 0, [2] * P, [1] * P)[r], g("ghost"))
+    rec(case, "add").check([a + b] * P)
+    if f"{case}/r0/ghost" in GOLD:
+        rec(case, "ghost").check(o.add_ghost_cells(al, 0, [2] * P, [1] * P))
 
 
 def stack_blocks(P, ny, nx, dtype):
@@ -125,8 +146,7 @@ def stack_blocks(P, ny, nx, dtype):
     return blocks, xg, yg
 
 
-@pytest.mark.parametrize("case", cases("stack", 4))
-def test_oracle_blockdiag_vstack_cgls(case):
+def stack_oracle(case):
     _, P, shp, dt = case.split("/")
     P, (ny, nx), dtype = int(P[1:]), tuple(int(v) for v in shp.split("x")), np.dtype(dt)
     blocks, xg, yg = stack_blocks(P, ny, nx, dtype)
@@ -144,15 +164,21 @@ def test_oracle_blockdiag_vstack_cgls(case):
     rmv = lambda v: o.SimArray(o.blockdiag(sblocks, v.locs, adjoint=True))   # noqa: E731
     xo, istop, iit, r1, r2, cost = o.cgls(mv, rmv, mv(o.SimArray(o.to_dist(xt, P))),
                                           o.SimArray(o.to_dist(np.zeros(P * nx, dtype=dtype), P)), niter=nx, tol=1e-5)
+    return P, y, xa, yv, xv, (xo.locs, istop, iit, r1, r2, np.asarray(cost))
+
+
+@pytest.mark.parametrize("case", cases("stack", 4))
+def test_oracle_blockdiag_vstack_cgls(case):
+    P, y, xa, yv, xv, (xo, istop, iit, r1, r2, cost) = stack_oracle(case)
+    rec(case, "bd_y").check(y, rtol=1e-13, atol=1e-13)
+    rec(case, "bd_xa").check(xa, rtol=1e-13, atol=1e-13)
+    rec(case, "vs_y").check(yv, rtol=1e-13, atol=1e-13)
+    rec(case, "vs_x").check([xv] * P, rtol=1e-12, atol=1e-12)
+    rec(case, "cgls_x").check(xo, rtol=1e-8, atol=1e-10)
+    rec(case, "cgls_cost").check([cost] * P, rtol=1e-7, atol=1e-12)
     for r in range(P):
         g = lambda n: GOLD[f"{case}/r{r}/{n}"]   # noqa: E731
-        np.testing.assert_allclose(y[r], g("bd_y"), rtol=1e-13, atol=1e-13)
-        np.testing.assert_allclose(xa[r], g("bd_xa"), rtol=1e-13, atol=1e-13)
-        np.testing.assert_allclose(yv[r], g("vs_y"), rtol=1e-13, atol=1e-13)
-        np.testing.assert_allclose(xv, g("vs_x"), rtol=1e-12, atol=1e-12)
         assert (iit, istop) == (int(g("cgls_iit")), int(g("cgls_istop")))
-        np.testing.assert_allclose(xo.locs[r], g("cgls_x"), rtol=1e-8, atol=1e-10)
-        np.testing.assert_allclose(cost, g("cgls_cost"), rtol=1e-7, atol=1e-12)
         np.testing.assert_allclose([r1, r2], [g("cgls_r1"), g("cgls_r2")], rtol=1e-6, atol=1e-14)
 
 
@@ -164,8 +190,7 @@ def mm_inputs(N, K, M, dtype):
     return A, X
 
 
-@pytest.mark.parametrize("case", cases("mm", 5))
-def test_oracle_matrixmult(case):
+def mm_oracle(case):
     _, P, shp, dt, kind = case.split("/")
     P, (N, K, M), dtype = int(P[1:]), tuple(int(v) for v in shp.split("x")), np.dtype(dt)
     A, X = mm_inputs(N, K, M, dtype)
@@ -181,11 +206,14 @@ def test_oracle_matrixmult(case):
         Xc = [X[:, (r // Pp) * bc:min(M, (r // Pp + 1) * bc)].flatten() for r in range(P)]
         y = o.blockmm_matvec(Arows, Xc, N, K, M, dtype=dtype)
         xa = o.blockmm_matvec(Arows, y, N, K, M, dtype=dtype, adjoint=True)
-    for r in range(P):
-        gy, gxa = GOLD[f"{case}/r{r}/y"], GOLD[f"{case}/r{r}/xa"]
-        np.testing.assert_allclose(y[r], gy, rtol=rtol)
-        if np.all(np.isfinite(gxa)):
-            np.testing.assert_allclose(xa[r], gxa, rtol=rtol * 10)
+    return y, xa, rtol
+
+
+@pytest.mark.parametrize("case", cases("mm", 5))
+def test_oracle_matrixmult(case):
+    y, xa, rtol = mm_oracle(case)
+    rec(case, "y").check(y, rtol=rtol)
+    rec(case, "xa").check(xa, rtol=rtol * 10)
 
 
 def fredholm_inputs(nz, dtype):
@@ -198,8 +226,7 @@ def fredholm_inputs(nz, dtype):
     return G.astype(dtype), x
 
 
-@pytest.mark.parametrize("case", cases("fredholm", 5))
-def test_oracle_fredholm(case):
+def fredholm_oracle(case):
     _, P, nz, dt, flags = case.split("/")
     P, nz, dtype = int(P[1:]), int(nz[2:]), np.dtype(dt)
     G, x = fredholm_inputs(nz, dtype)
@@ -207,8 +234,14 @@ def test_oracle_fredholm(case):
     off = np.cumsum([0] + ext)
     G_loc = [G[off[r]:off[r + 1]] for r in range(P)]
     y = o.fredholm1(G_loc, x, nz)
-    np.testing.assert_allclose(y, GOLD[case + "/y"], rtol=1e-13, atol=1e-13)
-    np.testing.assert_allclose(o.fredholm1(G_loc, y, nz, adjoint=True), GOLD[case + "/xa"], rtol=1e-12, atol=1e-12)
+    return y, o.fredholm1(G_loc, y, nz, adjoint=True)
+
+
+@pytest.mark.parametrize("case", cases("fredholm", 5))
+def test_oracle_fredholm(case):
+    y, xa = fredholm_oracle(case)
+    rec(case, "y").check(y, rtol=1e-13, atol=1e-13)
+    rec(case, "xa").check(xa, rtol=1e-12, atol=1e-12)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -228,13 +261,15 @@ def host(t):
 @pytest.mark.parametrize("case", [c for c in FD_CASES if c + "/reference_raises" not in KEYS])
 def test_gpu_first_derivative_vs_reference(pm, case):
     P, dims, h, kind, order, edge, dt = parse_fd(case)
-    x = GOLD[case + "/x"]
+    x, oy, oya = fd_oracle(case)
     Fop = pm.MPIFirstDerivative(dims, sampling=h, kind=kind, edge=edge, order=order, dtype=dt)
     xd = pm.DistributedArray.to_dist(x)
-    gy = np.concatenate([a.ravel() for a in ranks_of(case, "y")])
-    gya = np.concatenate([a.ravel() for a in ranks_of(case, "ya")])
-    np.testing.assert_allclose(host((Fop @ xd).asarray()), gy, rtol=1e-12, atol=1e-12)
-    np.testing.assert_allclose(host((Fop.H @ xd).asarray()), gya, rtol=1e-12, atol=1e-12)
+    y, ya = host((Fop @ xd).asarray()), host((Fop.H @ xd).asarray())
+    tol = dict(rtol=1e-12, atol=1e-12)
+    rec(case, "y").check(y, **tol)
+    rec(case, "ya").check(ya, **tol)
+    np.testing.assert_allclose(y, np.concatenate(oy), **tol)
+    np.testing.assert_allclose(ya, np.concatenate(oya), **tol)
 
 
 @pytest.mark.gpu
@@ -243,11 +278,12 @@ def test_gpu_config1_vs_reference(pm):
     x[5, 10] = 1.0
     Fop = pm.MPIFirstDerivative((11, 21), dtype=np.float64)
     y = Fop @ pm.DistributedArray.to_dist(x.ravel())
-    assert np.array_equal(host(y.asarray()).reshape(11, 21), GOLD["config1/y"])
+    GOLD.record("config1/y").check(host(y.asarray()).reshape(11, 21))
     xinv, istop, iit, r1, r2, cost = pm.cgls(Fop, y, x0=pm.DistributedArray.to_dist(np.zeros(231)), niter=10, tol=0.0)
     assert iit == int(GOLD["config1/iit"])
     np.testing.assert_allclose(cost, GOLD["config1/cost"], rtol=1e-6, atol=1e-12)
-    np.testing.assert_allclose(host(xinv.asarray()), GOLD["config1/xinv"], rtol=1e-6, atol=1e-9)
+    GOLD.record("config1/xinv").check(host(xinv.asarray()), rtol=1e-6, atol=1e-9)
+    np.testing.assert_allclose(host(xinv.asarray()), config1_oracle()[1], rtol=1e-6, atol=1e-9)
 
 
 @pytest.mark.gpu
@@ -258,14 +294,20 @@ def test_gpu_blockdiag_vstack_cgls_vs_reference(pm, case):
     blocks, xg, yg = stack_blocks(P, ny, nx, dtype)
     ops = [pm.MatrixMult(b) for b in blocks]                     # all P blocks on the one rank
     BD = pm.MPIBlockDiag(ops)
-    g = lambda n: np.concatenate([GOLD[f"{case}/r{r}/{n}"] for r in range(P)])   # noqa: E731
-    np.testing.assert_allclose(host((BD @ pm.DistributedArray.to_dist(xg)).asarray()), g("bd_y"), rtol=1e-12, atol=1e-12)
-    np.testing.assert_allclose(host((BD.H @ pm.DistributedArray.to_dist(yg)).asarray()), g("bd_xa"), rtol=1e-12, atol=1e-12)
+    _, oy, oxa, oyv, oxv, (oxo, *_o) = stack_oracle(case)
+    t12 = dict(rtol=1e-12, atol=1e-12)
+    for name, got, want in (("bd_y", host((BD @ pm.DistributedArray.to_dist(xg)).asarray()), oy),
+                            ("bd_xa", host((BD.H @ pm.DistributedArray.to_dist(yg)).asarray()), oxa)):
+        rec(case, name).check(got, **t12)
+        np.testing.assert_allclose(got, np.concatenate(want), **t12)
     VS = pm.MPIVStack(ops)
     xb = pm.DistributedArray.to_dist(xg[:nx], partition=pm.Partition.BROADCAST)
-    np.testing.assert_allclose(host((VS @ xb).asarray()), g("vs_y"), rtol=1e-12, atol=1e-12)
-    np.testing.assert_allclose(host((VS.H @ pm.DistributedArray.to_dist(yg)).asarray()), GOLD[f"{case}/r0/vs_x"],
-                               rtol=1e-11, atol=1e-11)
+    got = host((VS @ xb).asarray())
+    rec(case, "vs_y").check(got, **t12)
+    np.testing.assert_allclose(got, np.concatenate(oyv), **t12)
+    got = host((VS.H @ pm.DistributedArray.to_dist(yg)).asarray())
+    rec(case, "vs_x").check([got] * P, rtol=1e-11, atol=1e-11)
+    np.testing.assert_allclose(got, oxv, rtol=1e-11, atol=1e-11)
     sops = []
     for r in range(P):
         A = np.ones((ny, nx), dtype=dtype) * (r + 1)
@@ -276,8 +318,9 @@ def test_gpu_blockdiag_vstack_cgls_vs_reference(pm, case):
     xinv, istop, iit, r1, r2, cost = pm.cgls(Sop, yy, x0=pm.DistributedArray.to_dist(np.zeros(P * nx, dtype=dtype)),
                                              niter=nx, tol=1e-5)
     assert (iit, istop) == (int(GOLD[f"{case}/r0/cgls_iit"]), int(GOLD[f"{case}/r0/cgls_istop"]))
-    np.testing.assert_allclose(host(xinv.asarray()), g("cgls_x"), rtol=1e-6, atol=1e-8)
-    np.testing.assert_allclose(cost, GOLD[f"{case}/r0/cgls_cost"], rtol=1e-5, atol=1e-8)
+    rec(case, "cgls_x").check(host(xinv.asarray()), rtol=1e-6, atol=1e-8)
+    np.testing.assert_allclose(host(xinv.asarray()), np.concatenate(oxo), rtol=1e-6, atol=1e-8)
+    rec(case, "cgls_cost").check([np.asarray(cost)] * P, rtol=1e-5, atol=1e-8)
 
 
 @pytest.mark.gpu
@@ -288,9 +331,12 @@ def test_gpu_matrixmult_vs_reference(pm, case):
     A, X = mm_inputs(N, K, M, dtype)
     Aop = pm.MPIMatrixMult(A, M, kind=kind, dtype=dtype)
     y = Aop @ pm.DistributedArray.to_dist(X.ravel())
-    rtol = 1e-5 if dtype == np.float32 else 1e-13
-    np.testing.assert_allclose(host(y.asarray()), GOLD[f"{case}/r0/y"], rtol=rtol)
-    np.testing.assert_allclose(host((Aop.H @ y).asarray()), GOLD[f"{case}/r0/xa"], rtol=rtol * 10)
+    oy, oxa, rtol = mm_oracle(case)
+    got, gota = host(y.asarray()), host((Aop.H @ y).asarray())
+    rec(case, "y").check(got, rtol=rtol)
+    rec(case, "xa").check(gota, rtol=rtol * 10)
+    np.testing.assert_allclose(got, oy[0], rtol=rtol)
+    np.testing.assert_allclose(gota, oxa[0], rtol=rtol * 10)
 
 
 @pytest.mark.gpu
@@ -301,8 +347,12 @@ def test_gpu_fredholm_vs_reference(pm, case):
     G, x = fredholm_inputs(nz, dtype)
     Fop = pm.MPIFredholm1(G, nz=nz, dtype=dtype)
     y = Fop @ pm.DistributedArray.to_dist(x, partition=pm.Partition.BROADCAST)
-    np.testing.assert_allclose(host(y.asarray()), GOLD[case + "/y"], rtol=1e-12, atol=1e-12)
-    np.testing.assert_allclose(host((Fop.H @ y).asarray()), GOLD[case + "/xa"], rtol=1e-11, atol=1e-11)
+    oy, oxa = fredholm_oracle(case)
+    got, gota = host(y.asarray()), host((Fop.H @ y).asarray())
+    rec(case, "y").check(got, rtol=1e-12, atol=1e-12)
+    rec(case, "xa").check(gota, rtol=1e-11, atol=1e-11)
+    np.testing.assert_allclose(got, oy, rtol=1e-12, atol=1e-12)
+    np.testing.assert_allclose(gota, oxa, rtol=1e-11, atol=1e-11)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -316,6 +366,15 @@ def parse_sd(case):
     return int(P[1:]), ast.literal_eval(dims), float(h[1:]), kind, bool(int(e[1:])), np.dtype(dt)
 
 
+def sd_oracle(case):
+    P, dims, h, kind, edge, dt = parse_sd(case)
+    x = normal_input(9, int(np.prod(dims)), dt)
+    rec(case, "x").check(x)
+    y = o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, False, dtype=dt)
+    ya = o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, True, dtype=dt)
+    return x, y, ya
+
+
 @pytest.mark.parametrize("case", SD_CASES)
 def test_oracle_second_derivative(case):
     P, dims, h, kind, edge, dt = parse_sd(case)
@@ -325,25 +384,24 @@ def test_oracle_second_derivative(case):
             o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, False, dtype=dt)
             o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, True, dtype=dt)
         return
-    x = GOLD[case + "/x"]
-    y = o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, False, dtype=dt)
-    ya = o.second_derivative(o.to_dist(x, P), dims, h, kind, edge, True, dtype=dt)
-    for r, (gy, gya) in enumerate(zip(ranks_of(case, "y"), ranks_of(case, "ya"))):
-        np.testing.assert_array_equal(y[r], gy.ravel())
-        np.testing.assert_array_equal(ya[r], gya.ravel())
+    x, y, ya = sd_oracle(case)
+    rec(case, "y").check(y)
+    rec(case, "ya").check(ya)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", [c for c in SD_CASES if c + "/reference_raises" not in KEYS])
 def test_gpu_second_derivative_vs_reference(pm, case):
     P, dims, h, kind, edge, dt = parse_sd(case)
-    x = GOLD[case + "/x"]
+    x, oy, oya = sd_oracle(case)
     Sop = pm.MPISecondDerivative(dims, sampling=h, kind=kind, edge=edge, dtype=dt)
     xd = pm.DistributedArray.to_dist(x)
-    gy = np.concatenate([a.ravel() for a in ranks_of(case, "y")])
-    gya = np.concatenate([a.ravel() for a in ranks_of(case, "ya")])
-    np.testing.assert_allclose(host((Sop @ xd).asarray()), gy, rtol=1e-12, atol=1e-11)
-    np.testing.assert_allclose(host((Sop.H @ xd).asarray()), gya, rtol=1e-12, atol=1e-11)
+    y, ya = host((Sop @ xd).asarray()), host((Sop.H @ xd).asarray())
+    tol = dict(rtol=1e-12, atol=1e-11)
+    rec(case, "y").check(y, **tol)
+    rec(case, "ya").check(ya, **tol)
+    np.testing.assert_allclose(y, np.concatenate(oy), **tol)
+    np.testing.assert_allclose(ya, np.concatenate(oya), **tol)
 
 
 @pytest.mark.gpu
@@ -416,45 +474,56 @@ def test_next_fixture_inventory():
     assert len(GRAD_CASES) == 3 * 2 * 4 and len(LAP_CASES) == 3 * 4 * 3
 
 
+def grad_oracle(case):
+    P, dims, samp, kind, edge = parse_grad(case)
+    x = normal_input(13, int(np.prod(dims)), np.float64)
+    rec(case, "x").check([x] * P)
+    y = o.gradient(o.to_dist(x, P), dims, samp, kind, edge)
+    return x, y, o.gradient_adjoint(y, dims, samp, kind, edge)
+
+
 @pytest.mark.parametrize("case", GRAD_CASES)
 def test_oracle_gradient(case):
     P, dims, samp, kind, edge = parse_grad(case)
-    x = GOLD[case + "/r0/x"]
-    y = o.gradient(o.to_dist(x, P), dims, samp, kind, edge)
+    x, y, xa = grad_oracle(case)
     for ax in range(len(dims)):
-        for r, g in enumerate(ranks_of(case, f"y{ax}")):
-            np.testing.assert_allclose(y[ax][r], g.ravel(), rtol=1e-13, atol=1e-12)
-    xa = o.gradient_adjoint(y, dims, samp, kind, edge)
-    for r, g in enumerate(ranks_of(case, "xa")):
-        np.testing.assert_allclose(xa[r], g.ravel(), rtol=1e-13, atol=1e-11)
+        rec(case, f"y{ax}").check(y[ax], rtol=1e-13, atol=1e-12)
+    rec(case, "xa").check(xa, rtol=1e-13, atol=1e-11)
     flat = np.concatenate([np.concatenate(a) for a in y])
     np.testing.assert_allclose(np.dot(flat, flat), GOLD[case + "/r0/dot"], rtol=1e-13)
     np.testing.assert_allclose(np.linalg.norm(flat), GOLD[case + "/r0/norm"], rtol=1e-13)
 
 
-@pytest.mark.parametrize("case", LAP_CASES)
-def test_oracle_laplacian(case):
+def lap_oracle(case):
     P, dims, axes, weights, samp, kind, edge = parse_lap(case)
-    x = GOLD[case + "/r0/x"]
+    x = normal_input(14, int(np.prod(dims)), np.float64)
+    rec(case, "x").check([x] * P)
     y = o.laplacian(o.to_dist(x, P), dims, axes, weights, samp, kind, edge, False)
     ya = o.laplacian(o.to_dist(x, P), dims, axes, weights, samp, kind, edge, True)
-    for r, (g, ga) in enumerate(zip(ranks_of(case, "y"), ranks_of(case, "ya"))):
-        np.testing.assert_allclose(y[r], g.ravel(), rtol=1e-13, atol=1e-11)
-        np.testing.assert_allclose(ya[r], ga.ravel(), rtol=1e-13, atol=1e-11)
+    return x, y, ya
+
+
+@pytest.mark.parametrize("case", LAP_CASES)
+def test_oracle_laplacian(case):
+    x, y, ya = lap_oracle(case)
+    rec(case, "y").check(y, rtol=1e-13, atol=1e-11)
+    rec(case, "ya").check(ya, rtol=1e-13, atol=1e-11)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", GRAD_CASES)
 def test_gpu_gradient_vs_reference(pm, case):
     P, dims, samp, kind, edge = parse_grad(case)
-    x = GOLD[case + "/r0/x"]
+    x, oy, oxa = grad_oracle(case)
     Gop = pm.MPIGradient(dims, sampling=samp, kind=kind, edge=edge, dtype=np.float64)
     y = Gop.matvec(pm.DistributedArray.to_dist(x))
     for ax in range(len(dims)):
-        g = np.concatenate([a.ravel() for a in ranks_of(case, f"y{ax}")])
-        np.testing.assert_allclose(host(y[ax].asarray()), g, rtol=1e-12, atol=1e-11)
-    ga = np.concatenate([a.ravel() for a in ranks_of(case, "xa")])
-    np.testing.assert_allclose(host(Gop.rmatvec(y).asarray()), ga, rtol=1e-12, atol=1e-10)
+        got = host(y[ax].asarray())
+        rec(case, f"y{ax}").check(got, rtol=1e-12, atol=1e-11)
+        np.testing.assert_allclose(got, np.concatenate(oy[ax]), rtol=1e-12, atol=1e-11)
+    got = host(Gop.rmatvec(y).asarray())
+    rec(case, "xa").check(got, rtol=1e-12, atol=1e-10)
+    np.testing.assert_allclose(got, np.concatenate(oxa), rtol=1e-12, atol=1e-10)
     np.testing.assert_allclose(y.dot(y), GOLD[case + "/r0/dot"], rtol=1e-12)
     np.testing.assert_allclose(y.norm(), GOLD[case + "/r0/norm"], rtol=1e-12)
 
@@ -463,13 +532,13 @@ def test_gpu_gradient_vs_reference(pm, case):
 @pytest.mark.parametrize("case", LAP_CASES)
 def test_gpu_laplacian_vs_reference(pm, case):
     P, dims, axes, weights, samp, kind, edge = parse_lap(case)
-    x = GOLD[case + "/r0/x"]
+    x, oy, oya = lap_oracle(case)
     Lop = pm.MPILaplacian(dims, axes=axes, weights=weights, sampling=samp, kind=kind, edge=edge, dtype=np.float64)
     xd = pm.DistributedArray.to_dist(x)
-    g = np.concatenate([a.ravel() for a in ranks_of(case, "y")])
-    ga = np.concatenate([a.ravel() for a in ranks_of(case, "ya")])
-    np.testing.assert_allclose(host((Lop @ xd).asarray()), g, rtol=1e-12, atol=1e-10)
-    np.testing.assert_allclose(host((Lop.H @ xd).asarray()), ga, rtol=1e-12, atol=1e-10)
+    tol = dict(rtol=1e-12, atol=1e-10)
+    for name, got, want in (("y", host((Lop @ xd).asarray()), oy), ("ya", host((Lop.H @ xd).asarray()), oya)):
+        rec(case, name).check(got, **tol)
+        np.testing.assert_allclose(got, np.concatenate(want), **tol)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -555,9 +624,16 @@ MDC_CASES = cases("mdc", 5)
 def mdc_inputs(case):
     _, P, t, dt, cp = case.split("/")
     P, twosided, conj, prescaled = int(P[1:]), bool(int(t[1:])), bool(int(cp[1])), bool(int(cp[3]))
-    G, m, d = GOLD[case + "/G"], GOLD[case + "/m"], GOLD[case + "/d"]
-    nt = 31 if twosided else 32
-    nf = G.shape[0]
+    dtype = np.dtype(dt)
+    rng = np.random.default_rng(31)          # drawn as make_golden.t_mdc draws them
+    ns, nr, nv, nt = 6, 5, 3, (31 if twosided else 32)
+    nf = int(np.ceil((nt + 1) / 2)) - 3
+    G = (rng.standard_normal((nf, ns, nr)) + 1j * rng.standard_normal((nf, ns, nr))).astype(dtype)
+    rdt = np.real(np.ones(1, dtype)).dtype
+    m = rng.standard_normal(nt * nr * nv).astype(rdt)
+    d = rng.standard_normal(nt * ns * nv).astype(rdt)
+    for name, a in (("G", G), ("m", m), ("d", d)):
+        rec(case, name).check(a)
     off = np.cumsum([0] + [nf // P + (1 if r < nf % P else 0) for r in range(P)])
     return P, twosided, conj, prescaled, G, m, d, nt, off
 
@@ -566,18 +642,22 @@ def test_mdc_inventory():
     assert len(MDC_CASES) == 3 * 2 * 3
 
 
-@pytest.mark.parametrize("case", MDC_CASES)
-def test_oracle_mdc(case):
+def mdc_oracle(case):
     P, twosided, conj, prescaled, G, m, d, nt, off = mdc_inputs(case)
     Gl = [G[off[r]:off[r + 1]].astype(np.complex128) for r in range(P)]
     kw = dict(dt=0.004, dr=2.0, prescaled=prescaled, conj=conj)
-    y = o.mdc(Gl, m.astype(np.float64), nt, 3, twosided, False, **kw)
-    xa = o.mdc(Gl, d.astype(np.float64), nt, 3, twosided, True, **kw)
-    gy, gxa = GOLD[case + "/y"], GOLD[case + "/xa"]
-    assert np.abs(gy.imag).max() == 0 and np.abs(gxa.imag).max() == 0
+    return o.mdc(Gl, m.astype(np.float64), nt, 3, twosided, False, **kw), o.mdc(Gl, d.astype(np.float64), nt, 3, twosided, True, **kw)
+
+
+@pytest.mark.parametrize("case", MDC_CASES)
+def test_oracle_mdc(case):
+    G = mdc_inputs(case)[4]
+    y, xa = mdc_oracle(case)
+    gy, gxa = rec(case, "y"), rec(case, "xa")
+    assert gy.imag_zero and gxa.imag_zero
     tol = 2e-6 if G.dtype == np.complex64 else 1e-13
-    np.testing.assert_allclose(y, gy.real, rtol=tol, atol=tol * np.abs(gy).max())
-    np.testing.assert_allclose(xa, gxa.real, rtol=tol, atol=tol * np.abs(gxa).max())
+    gy.check(y, rtol=tol, atol=tol * gy.amax)
+    gxa.check(xa, rtol=tol, atol=tol * gxa.amax)
 
 
 @pytest.mark.gpu
@@ -587,7 +667,9 @@ def test_gpu_mdc_vs_reference(pm, case):
     Mop = pm.MPIMDC(G, nt=nt, nv=3, nfreq=G.shape[0], dt=0.004, dr=2.0, twosided=twosided, conj=conj, prescaled=prescaled)
     y = Mop @ pm.DistributedArray.to_dist(m, partition=pm.Partition.BROADCAST)
     xa = Mop.H @ pm.DistributedArray.to_dist(d, partition=pm.Partition.BROADCAST)
-    gy, gxa = GOLD[case + "/y"].real, GOLD[case + "/xa"].real
+    oy, oxa = mdc_oracle(case)
     tol = 2e-4 if G.dtype == np.complex64 else 1e-11
-    np.testing.assert_allclose(host(y.asarray()).real, gy, rtol=tol, atol=tol * np.abs(gy).max())
-    np.testing.assert_allclose(host(xa.asarray()).real, gxa, rtol=tol, atol=tol * np.abs(gxa).max())
+    for name, got, want in (("y", host(y.asarray()).real, oy), ("xa", host(xa.asarray()).real, oxa)):
+        g = rec(case, name)
+        g.check(got, rtol=tol, atol=tol * g.amax)
+        np.testing.assert_allclose(got, want, rtol=tol, atol=tol * g.amax)
