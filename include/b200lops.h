@@ -146,6 +146,17 @@ int b2_second_derivative_halo(int kind, int edge, int adjoint, int* need_lo, int
 int b2_derivative_axis(b2_ctx* ctx, const void* x, void* y, size_t n_outer, size_t n_axis, size_t n_inner,
                        int deriv, int kind, int order, int edge, double sampling, int adjoint, int dtype,
                        void* stream);
+/* rank-local 1-D convolution with a real filter along the MIDDLE axis of a C-ordered [n_outer][n_axis][n_inner]
+ * block: the pylops.signalprocessing.Convolve1D that MPIBlockDiag applies per rank (tutorials/reflectivity.py:75,
+ * basicoperators/BlockDiag.py:127-129).  taps: nh DEVICE values of the data's precision (dtype B2_F32 | B2_F64;
+ * complex data: pass the real dtype with the (re, im) pairs folded into n_inner).  Zero outside [0, n_axis):
+ *   forward:  y[i] = sum_k taps[k] x[i + offset - k]
+ *   adjoint:  y[j] = sum_k taps[k] x[j - offset + k]     (the exact transpose)
+ * Any offset; 1 <= nh <= B2_CONV_MAX_TAPS (else B2_ERR_UNSUPPORTED).  x and y must not overlap.  Each output sums
+ * its taps in a fixed order in the data's precision: results are identical from run to run. */
+#define B2_CONV_MAX_TAPS 2048
+int b2_convolve1d(b2_ctx* ctx, const void* x, void* y, size_t n_outer, size_t n_axis, size_t n_inner,
+                  const void* taps, int nh, long long offset, int adjoint, int dtype, void* stream);
 /* Peer-memory halo exchange fused INTO the stencil kernel (replaces the add_ghost_cells Send/Recv pairs of
  * DistributedArray.py:876-953 as used by FirstDerivative.py:221-247, 276-319 and SecondDerivative.py): every rank
  * owns a box of b2_halo_bytes(cap) bytes in IPC-mapped memory (b2_symm_alloc + b2_ipc_*); boxes_host[r] is rank r's

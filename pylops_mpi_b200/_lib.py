@@ -86,6 +86,7 @@ def _load():
         "b2_second_derivative": ([vp, vp, vp, vp, i, vp, i, sz, sz, sz, sz, i, i, d, i, i, vp], i),
         "b2_second_derivative_halo": ([i, i, i, C.POINTER(i), C.POINTER(i)], i),
         "b2_derivative_axis": ([vp, vp, vp, sz, sz, sz, i, i, i, i, d, i, i, vp], i),
+        "b2_convolve1d": ([vp, vp, vp, sz, sz, sz, vp, i, C.c_longlong, i, i, vp], i),
         "b2_halo_bytes": ([sz], sz),
         "b2_halo_create": ([i, i, C.POINTER(vp), sz, C.POINTER(vp)], i),
         "b2_halo_destroy": ([vp], i),

@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libb200lops.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
-SOURCES = ["ctx.cu", "elementwise.cu", "reduce.cu", "sparsity.cu", "stencil.cu", "gemv.cu", "gemm_simt.cu",
+SOURCES = ["ctx.cu", "elementwise.cu", "reduce.cu", "sparsity.cu", "stencil.cu", "convolve.cu", "gemv.cu", "gemm_simt.cu",
            "gemm_tc.cu", "gemm_tc2.cu", "fredholm_tc.cu", "host_pipe.cu", "comm.cu", "peer.cu"]
 
 

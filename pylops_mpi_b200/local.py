@@ -215,6 +215,85 @@ class SecondDerivative(_AxisDerivative):
         super().__init__(dims, axis=axis, sampling=sampling, kind=kind, edge=edge, order=3, dtype=dtype)
 
 
+CONVOLVE_MAX_TAPS = 2048       # B2_CONV_MAX_TAPS (include/b200lops.h)
+
+
+class Convolve1D(LocalOperator):
+    """Rank-local 1-D convolution of a C-ordered ``dims`` block with a real filter ``h`` along ``axis`` -- the
+    ``pylops.signalprocessing.Convolve1D(dims, h, offset, axis)`` that the seismic tutorials wrap in MPIBlockDiag
+    (tutorials/reflectivity.py:75)::
+
+        y[i] = sum_k h[k] x[i + offset - k]        (x = 0 outside the axis)
+
+    and its exact transpose.  One batched launch per apply (b2_convolve1d); the taps are uploaded once, here.
+    ``method`` is accepted for signature compatibility: "direct", "fft" and "overlapadd" all run the direct
+    kernel.  Complex data is convolved with the real filter (real and imaginary parts alike)."""
+
+    def __init__(self, dims, h, offset: int = 0, axis: int = -1, dtype="float64", method=None):
+        if method not in (None, "direct", "fft", "overlapadd"):
+            raise NotImplementedError("method must be None, 'direct', 'fft' or 'overlapadd'")
+        if isinstance(h, torch.Tensor):
+            h = h.detach().cpu().numpy()
+        h = np.asarray(h)
+        if np.iscomplexobj(h):
+            raise NotImplementedError("complex filters are not supported")
+        if h.ndim != 1:
+            raise NotImplementedError("only a single 1-D filter is supported (no per-trace filters)")
+        if not 1 <= h.size <= CONVOLVE_MAX_TAPS:
+            raise NotImplementedError(f"filter length must be between 1 and {CONVOLVE_MAX_TAPS}, got {h.size}")
+        self.dims = tuple(int(d) for d in (dims if np.ndim(dims) else (dims,)))
+        self.axis = axis % len(self.dims)
+        n = int(np.prod(self.dims))
+        self.shape = (n, n)
+        self.nh, self.offset = int(h.size), int(offset)
+        self._tdtype = _lib.torch_dtype(dtype)
+        if _REAL_OF.get(self._tdtype, self._tdtype) not in (torch.float32, torch.float64):
+            raise NotImplementedError(f"dtype {dtype} is not supported (float32, float64, complex64, complex128)")
+        self.dtype = _lib.numpy_dtype(self._tdtype)
+        _lib.ctx()
+        # taps in both precisions (data of either precision may arrive), so an apply never copies from the host
+        self._taps = {t: torch.as_tensor(h.astype(_lib.numpy_dtype(t))).to("cuda") for t in (torch.float32, torch.float64)}
+        self.n_outer = int(np.prod(self.dims[:self.axis])) if self.axis else 1
+        self.n_axis = self.dims[self.axis]
+        self.n_inner = int(np.prod(self.dims[self.axis + 1:])) if self.axis + 1 < len(self.dims) else 1
+
+    def _apply(self, x: torch.Tensor, adjoint: int, out=None) -> torch.Tensor:
+        x = x.reshape(-1)
+        if x.numel() != self.shape[1]:
+            raise ValueError(f"dimension mismatch: operator {self.shape}, vector {x.numel()}")
+        tdt = self._tdtype
+        if x.dtype.is_complex and not tdt.is_complex:
+            tdt = _CPLX_OF[torch.promote_types(tdt, _REAL_OF[x.dtype])]     # real taps on complex data
+        if x.dtype != tdt:
+            x = x.to(tdt)
+        if not x.is_contiguous():
+            x = x.contiguous()
+        direct = out is not None and out.dtype == tdt and out.is_contiguous() and out.numel() == x.numel()
+        y = out if direct else torch.empty_like(x)
+        real = _REAL_OF.get(tdt, tdt)
+        # complex data: the (re, im) pairs are part of the inner dimension
+        n_inner = 2 * self.n_inner if tdt.is_complex else self.n_inner
+        taps = self._taps[real]
+        _lib.check(_lib.lib.b2_convolve1d(_lib.ctx(), x.data_ptr(), y.data_ptr(), self.n_outer, self.n_axis, n_inner,
+                                          taps.data_ptr(), self.nh, self.offset, adjoint, _lib.code(real),
+                                          _lib.stream()), "b2_convolve1d")
+        if out is not None and not direct:
+            return _store(out, y)
+        return y
+
+    def _matvec(self, x, out=None):
+        return self._apply(x, 0, out)
+
+    def _rmatvec(self, x, out=None):
+        return self._apply(x, 1, out)
+
+    def matvec(self, x, out=None):
+        return self._apply(x, 0, out)
+
+    def rmatvec(self, x, out=None):
+        return self._apply(x, 1, out)
+
+
 class FFT(LocalOperator):
     """Rank-local real FFT along ``axis`` of a ``dims`` block -- the role of third-party
     ``pylops.signalprocessing.FFT(dims, axis, real=True, ifftshift_before=..., norm="ortho")`` inside

@@ -48,7 +48,7 @@ class Solver:
 _GRAPH_SAFE_TYPES = ("MPIBlockDiag", "MPIVStack", "MPIHStack", "MPIFirstDerivative", "MPISecondDerivative",
                      "_MPISummaMatrixMult", "_MPIBlockMatrixMult", "_AdjointLinearOperator", "_TransposedLinearOperator",
                      "_ProductLinearOperator", "_ScaledLinearOperator", "_SumLinearOperator", "_ConjLinearOperator",
-                     "MatrixMult", "FirstDerivative", "SecondDerivative")
+                     "MatrixMult", "FirstDerivative", "SecondDerivative", "Convolve1D")
 
 
 _GRAPH_POOL = {}
